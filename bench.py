@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark (driver contract): samples/sec of the launched DDP training job.
 
-    python bench.py --gpus N --steps K --warmup W [--model gpt2|bert|resnet50|mnist]
+    python bench.py --gpus N --steps K --warmup W [--model gpt2|bert|resnet50|mnist] [--dump-outputs DIR]
 
 * ``value``  -- device-timed (CUDA events, max over ranks) whole-job samples/sec of the flagship
   training step (GPT-2 small, seq 1024, bf16, per-GPU batch 16 = weak scaling) run by the ranks the
@@ -11,6 +11,12 @@
   control plane (API server + node agent + operator), ``apply``-s an ``AITrainingJob`` with N replicas
   and reads the samples/sec its controller-launched workers report (fresh processes, one per GPU,
   pinned with CUDA_VISIBLE_DEVICES, NCCL over NVLink); also reports reconcile->running latency.
+* ``--dump-outputs DIR`` -- after the timed steps, rank 0 of the device-timed run writes what its last step computed:
+  ``loss.npy`` and a fixed sample of the trained fp32 parameters and AdamW moments (``params.npy``, ``exp_avg.npy``,
+  ``exp_avg_sq.npy``; float32, 48 MB at most).  Inputs and initial weights are seeded, so two builds run with the same
+  arguments can be compared output for output -- within a tolerance: the fp32 atomic accumulations of the kernels
+  (split-K weight gradients, bias column sums, the gradient norm) repeat to round-off, not bit for bit, and AdamW
+  carries that into the weights, so two runs of one build on the GPU already differ slightly.
 * ``--impl reference`` -- the reference is a Go Kubernetes operator with no Python package, no GPU
   code and no cluster to run against here: prints ``{"impl": "reference", "unavailable": ...}``.
 
@@ -101,7 +107,7 @@ class ClockSampler:
                 "scope": scope}
 
 
-def worker_args(a, result_path=""):
+def worker_args(a, result_path="", dump_dir=""):
     from trainingjob_operator_b200.runtime import worker
 
     d = MODEL_DEFAULTS[a.model]
@@ -111,6 +117,8 @@ def worker_args(a, result_path=""):
         argv.append("--no-graph")
     if result_path:
         argv += ["--result", result_path]
+    if dump_dir:
+        argv += ["--dump-outputs", dump_dir]
     return worker.parse_args(argv), argv
 
 
@@ -124,7 +132,7 @@ def run_device_timed(a):
     os.environ.setdefault("MASTER_PORT", "29511")
     os.environ.pop("AITJ_MASTER", None)
     rank = int(os.environ["RANK"])
-    wa, _ = worker_args(a)
+    wa, _ = worker_args(a, dump_dir=a.dump_outputs)
     sampler = ClockSampler() if rank == 0 else None
     if sampler:
         sampler.start()
@@ -247,7 +255,11 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-warm-pool", action="store_true", help="e2e arm: cold worker start instead of the agent's warm pool")
     ap.add_argument("--e2e-timeout", type=float, default=900.0)
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the last timed step's loss and a sample of the trained state to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.warmup = max(3, a.warmup)
 
     if a.impl == "reference":
@@ -268,7 +280,10 @@ def main():
 
     d = MODEL_DEFAULTS[a.model]
     res, clocks = run_device_timed(a)
-    done_flag = os.path.join(tempfile.gettempdir(), f"aitj_bench_done_{os.environ.get('MASTER_PORT', '0')}")
+    # per user: the flag outlives the run, and another user's flag in a shared temp directory can be neither removed nor
+    # overwritten
+    done_flag = os.path.join(tempfile.gettempdir(),
+                             f"aitj_bench_done_{os.getuid()}_{os.environ.get('MASTER_PORT', '0')}")
     if rank != 0:
         # keep the process (and torchrun) alive while rank 0 measures the end-to-end path
         import torch

@@ -1,26 +1,20 @@
-"""API-surface parity with the reference, checked mechanically against its sources when they are present
-(``/root/reference``; skipped elsewhere, e.g. on the GPU box): every JSON field of its Go API types, every string constant
-of its API package and every command-line flag of its options exists here under the same spelling."""
+"""API-surface parity with the reference, checked mechanically against a recording of its sources
+(``tests/golden/reference_api.json``, written by ``tools/record_reference_api.py``): every JSON field of its Go API types,
+every string constant of its API package and every command-line flag of its options exists here under the same spelling."""
 import dataclasses
-import glob
+import hashlib
+import json
 import os
-import re
 
-import pytest
-
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "pkg", "apis")), reason="reference sources not present")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REF = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_api.json")))
 
 
 def test_every_json_field_of_the_reference_api_types_exists():
     """types.go:29-152, replica.go:9-63 -- byte-compatible spellings incl. ``RestartCount`` and phase ``Succeed``."""
     from trainingjob_operator_b200.api import types as T
 
-    tags = set()
-    for f in glob.glob(os.path.join(REF, "pkg/apis/aitrainingjob/v1/*.go")):
-        if "zz_generated" not in f:
-            tags |= set(re.findall(r'json:"([^",]+)', open(f).read()))
+    tags = set(REF["json_fields"])
     ours = set()
     for name in dir(T):
         c = getattr(T, name)
@@ -30,10 +24,7 @@ def test_every_json_field_of_the_reference_api_types_exists():
 
 
 def test_every_string_constant_of_the_reference_api_package_exists():
-    ref = set()
-    for f in glob.glob(os.path.join(REF, "pkg/apis/aitrainingjob/v1/*.go")):
-        if "zz_generated" not in f:
-            ref |= set(re.findall(r'\b\w+(?:\s+\w+)?\s*=\s*"([^"]+)"', open(f).read()))
+    ref = set(REF["string_constants"])
     ours = open(os.path.join(ROOT, "trainingjob_operator_b200/api/constants.py")).read() + \
         open(os.path.join(ROOT, "trainingjob_operator_b200/api/types.py")).read()
     missing = [c for c in sorted(ref) if f'"{c}"' not in ours and f"'{c}'" not in ours]
@@ -42,8 +33,7 @@ def test_every_string_constant_of_the_reference_api_package_exists():
 
 def test_every_command_line_flag_of_the_reference_exists():
     """cmd/app/options/options.go:61-72 (+ the leader-election set bound by leaderelectionconfig.BindFlags)."""
-    src = open(os.path.join(REF, "cmd/app/options/options.go")).read()
-    flags = set(re.findall(r'fs\.\w+\([^"]*"([\w-]+)"', src))
+    flags = set(REF["flags"])
     ours = open(os.path.join(ROOT, "trainingjob_operator_b200/cmd/options.py")).read()
     missing = [f for f in sorted(flags) if f"--{f}" not in ours and f'"{f}"' not in ours]
     assert len(flags) >= 9 and not missing, missing
@@ -52,5 +42,5 @@ def test_every_command_line_flag_of_the_reference_exists():
 
 
 def test_the_reference_example_is_shipped_verbatim():
-    assert open(os.path.join(REF, "example/paddle-mnist.yaml")).read() == \
-        open(os.path.join(ROOT, "examples/paddle-mnist.yaml")).read()
+    ours = open(os.path.join(ROOT, "examples/paddle-mnist.yaml"), "rb").read()
+    assert hashlib.sha256(ours).hexdigest() == REF["example_paddle_mnist_sha256"]

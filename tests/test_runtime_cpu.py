@@ -491,3 +491,28 @@ def test_nn_module_workers_step_on_cpu(name, batch, params):
     ad.train_step()
     assert any(not torch.equal(a, b) for a, b in zip(snap, state))       # the state tensors ARE the live state
     ad.after_state_load()
+
+
+def test_bench_dump_outputs_are_the_same_for_the_same_arguments(tmp_path):
+    """``bench.py --dump-outputs``: the last timed step's loss and the trained state land as float32 ``.npy`` files within
+    64 MB, and two runs with the same arguments write the same values (seeded inputs and initial weights)."""
+    import json
+
+    import numpy as np
+
+    dumps = []
+    for run in ("a", "b"):
+        out = tmp_path / run
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--model", "mnist", "--batch", "8", "--steps",
+                            "2", "--warmup", "3", "--no-e2e", "--dump-outputs", str(out)], cwd=str(tmp_path),
+                           env=dict(os.environ, OMP_NUM_THREADS="2", CUDA_VISIBLE_DEVICES=""),   # CPU: bitwise repeatable
+                           capture_output=True, text=True, timeout=300)
+        assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
+        line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+        assert line["steps"] == 2
+        dumps.append({f.name: np.load(f) for f in sorted(out.iterdir())})
+    a, b = dumps
+    assert sorted(a) == ["exp_avg.npy", "exp_avg_sq.npy", "loss.npy", "params.npy"]
+    assert all(v.dtype == np.float32 and np.isfinite(v).all() for v in a.values())
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    assert all(np.array_equal(a[k], b[k]) for k in a)

@@ -142,8 +142,9 @@ static void stress_store_cascade() {
   Store s("", 1 << 16);
   std::atomic<bool> stop{false};
   std::atomic<long> events{0};
+  // opened before any writer starts: a watch opened at "now" sees nothing published before it
+  const int64_t id = s.watch_open("Pod", "", 0);
   std::thread watcher([&] {
-    int64_t id = s.watch_open("Pod", "", 0);
     while (!stop.load()) events += static_cast<long>(s.watch_next_many(id, 0.02, 32).size());
     for (;;) {
       auto batch = s.watch_next_many(id, 0.0, 64, false);

@@ -138,6 +138,7 @@ class TorchAdapter:
 
         self.name, self.batch, self.dev, self.args = name, batch, device, args
         g = torch.Generator().manual_seed(args.seed + 1)
+        torch.manual_seed(args.seed)       # the modules below draw their initial weights from the global generator
         if name == "mnist":
             self.module = MnistCNN()
             shape, ncls = (1, 28, 28), 10
@@ -151,7 +152,6 @@ class TorchAdapter:
             shape, ncls = (64,), 10
         else:
             raise ValueError(name)
-        torch.manual_seed(args.seed)
         self.module = self.module.to(device)
         self.channels_last = device.type == "cuda" and len(shape) == 3
         if self.channels_last:
@@ -346,6 +346,26 @@ def guarded(breaker, generation: int, fn):
     if breaker.tripped:
         raise RuntimeError("the communicator was aborted while the state hand-off was in flight")
     return out
+
+
+# ------------------------------------------------------------------------------------ outputs
+DUMP_SAMPLE = 1 << 22      # elements kept per state tensor: 3 x 16 MB for GPT-2 small's parameters and AdamW moments
+
+
+def dump_outputs(out_dir: str, loss: float, state: List[torch.Tensor]) -> None:
+    """What the last training step produced, as ``out_dir/<name>.npy`` (float32): its loss and the trained state (fp32
+    parameters, then the optimizer's moments).  A tensor larger than ``DUMP_SAMPLE`` elements is cut to a fixed sample
+    (sorted indices from a generator seeded with 0), so that runs of two builds on the same inputs compare element for
+    element."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([loss], dtype=np.float32))
+    for name, t in zip(("params", "exp_avg", "exp_avg_sq"), state):
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randint(0, t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0))
+            t = t.index_select(0, idx.sort().values.to(t.device))
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------ main loop
@@ -669,6 +689,10 @@ def run(args) -> Dict[str, Any]:
             or getattr(adapter, "graph_error", None),
             "allreduce": getattr(getattr(adapter, "trainer", None), "allreduce_backend", "nccl" if world > 1 else "none"),
         })
+        if args.dump_outputs:
+            adapter.prepare_state()         # collective: the whole trained state on every rank
+            if rank == 0:
+                dump_outputs(args.dump_outputs, losses[-1], adapter.state_tensors())
     if rank == 0 and args.result:
         os.makedirs(os.path.dirname(os.path.abspath(args.result)), exist_ok=True)
         with open(args.result + ".tmp", "w") as f:
@@ -701,6 +725,8 @@ def parse_args(argv=None):
     ap.add_argument("--ckpt-dir", default="")
     ap.add_argument("--ckpt-every", type=int, default=0)
     ap.add_argument("--step-sleep", type=float, default=0.0)
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the last step's loss and a sample of the trained state to DIR")
     return ap.parse_args(argv)
 
 
